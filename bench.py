@@ -38,6 +38,7 @@ sys.path.insert(0, str(ROOT))
 METRIC = "QPS @ recall@10 (HNSW selective recompute, all-MiniLM-L6-v2 384d, efSearch=64, k=10)"
 WORLD_VERSION = "w4"  # bump when the corpus generator / graph builder changes what a cached world holds
 K = 10
+DUMP_QUERIES = 1024  # queries per step per GPU of a --dump-outputs run without --queries
 
 
 def parse():
@@ -48,7 +49,8 @@ def parse():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--chunks", type=int, default=int(os.environ.get("LB2_BENCH_CHUNKS", 10_000_000)))
     ap.add_argument("--queries", type=int, default=int(os.environ.get("LB2_BENCH_QUERIES", 0)),
-                    help="queries per step per GPU; 0 = sized from --budget-s after a calibration call")
+                    help="queries per step per GPU; 0 = sized from --budget-s after a calibration call "
+                         f"({DUMP_QUERIES} with --dump-outputs, so that the inputs do not depend on a timing)")
     ap.add_argument("--budget-s", type=float, default=float(os.environ.get("LB2_BENCH_BUDGET_S", 300)),
                     help="wall budget of the warm-up + timed steps (sizes --queries when that is 0)")
     ap.add_argument("--ref-budget-s", type=float, default=float(os.environ.get("LB2_BENCH_REF_BUDGET_S", 300)),
@@ -67,6 +69,8 @@ def parse():
     ap.add_argument("--extras", action="store_true", help="call-scope de-duplication and stored-vector (traversal-only) side measurements")
     ap.add_argument("--diskann", action="store_true", help="extra: the DiskANN/Vamana path over the same corpus")
     ap.add_argument("--rebuild", action="store_true", help="ignore a cached world")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one returned to the "
+                    "caller as DIR/labels.npy (float64 passage ids, -1 = none) and DIR/distances.npy (float32), [queries, k]")
     return ap.parse_args()
 
 
@@ -329,6 +333,8 @@ def run_b200(args):
     # ---- size the step from the wall budget: one calibration call of 256 queries per GPU
     Qpool = np.ascontiguousarray(W["Q"])
     nq = args.queries
+    if nq <= 0 and args.dump_outputs:
+        nq = min(DUMP_QUERIES, P // world)
     if nq <= 0:
         ncal = 256
         qc = Qpool[np.arange(world * ncal) % P]
@@ -380,6 +386,8 @@ def run_b200(args):
     barrier()
     t_wall = time.perf_counter() - t_begin
     clk = clocks.stop()
+    if args.dump_outputs and rank == 0 and args.steps > 0:
+        dump_outputs(Path(args.dump_outputs), out)
     red = torch.tensor([agg["gpu_ms"] / 1e3, t_calls, t_wall], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(red, op=dist.ReduceOp.MAX)
@@ -475,6 +483,14 @@ def run_b200(args):
         dist.destroy_process_group()
     if out is not None:
         emit(REAL_STDOUT, out)
+
+
+def dump_outputs(d: Path, out):
+    """The last timed step's result, as the caller received it (all ranks' queries: the results are gathered)."""
+    d.mkdir(parents=True, exist_ok=True)
+    np.save(d / "labels.npy", np.array([[int(x) for x in row] for row in out["labels"]], np.float64))
+    np.save(d / "distances.npy", np.asarray(out["distances"], np.float32))
+    log(f"outputs of the last timed step written to {d}")
 
 
 def compare_results(I_gpu, D_gpu, I_ref, D_ref):

@@ -8,6 +8,7 @@
 from __future__ import annotations
 
 import ctypes as C
+import os
 import subprocess
 from pathlib import Path
 
@@ -18,9 +19,12 @@ DIST_CB = C.CFUNCTYPE(None, C.c_void_p, C.POINTER(C.c_float), C.c_int64, C.POINT
 
 
 def build(ref: bool = True) -> None:
+    """liboracle.so, and oracle/_ref/ where the original LEANN's sources can be read: at the Makefile's REF, or at
+    $LEANN_REFERENCE when that is set."""
     subprocess.run(["make", "-s", "-C", str(HERE), "all"], check=True)
-    if ref and Path("/root/reference/packages/leann-backend-hnsw/third_party/faiss").exists():
-        subprocess.run(["make", "-s", "-j8", "-C", str(HERE), "ref"], check=True)
+    src = [f"REF={os.environ['LEANN_REFERENCE']}"] if os.environ.get("LEANN_REFERENCE") else []
+    if ref and subprocess.run(["make", "-s", "-C", str(HERE), "have-ref", *src], capture_output=True).returncode == 0:
+        subprocess.run(["make", "-s", "-j8", "-C", str(HERE), "ref", *src], check=True)
 
 
 def _p(a, t):

@@ -206,12 +206,28 @@ class DiskannPrimitives:
             raise RuntimeError("reference load_pq_centroid_bin failed")
         return C.c_void_p(h)
 
+    def pq_num_chunks(self, table) -> int:
+        return int(self.lib.dref_pq_num_chunks(table))
+
     def lut(self, table, qvec_prepared, n_chunks):
         qv = np.ascontiguousarray(qvec_prepared, np.float32).copy()
         self.lib.dref_pq_preprocess_query(table, _p(qv, C.c_float))
         lut = np.empty((n_chunks, 256), np.float32)
         self.lib.dref_pq_populate_chunk_distances(table, _p(qv, C.c_float), _p(lut, C.c_float))
         return qv, lut
+
+    class QueryTable:
+        """preprocess_query + populate_chunk_distances for one query, then pq_dist_lookup against that table."""
+
+        def __init__(self, prims, table, qvec_prepared, n_chunks):
+            self.prims = prims
+            _, self.lut = prims.lut(table, qvec_prepared, n_chunks)
+
+        def dists(self, ids, codes):
+            return self.prims.pq_dists(self.lut, ids, codes)
+
+    def query_table(self, table, qvec_prepared, n_chunks):
+        return DiskannPrimitives.QueryTable(self, table, qvec_prepared, n_chunks)
 
     def pq_dists(self, lut, ids, codes):
         ids = np.ascontiguousarray(ids, np.uint32)

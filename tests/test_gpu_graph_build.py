@@ -8,6 +8,8 @@ pytestmark = pytest.mark.gpu
 
 torch = pytest.importorskip("torch")
 
+from helpers import reference  # noqa: E402,F401  (fixture)
+
 
 def clustered(n, d, n_clusters, seed, spread=0.35):
     rng = np.random.default_rng(seed)
@@ -149,28 +151,41 @@ def test_incremental_builder_matches_the_exact_builder(tmp_path):
     assert r_inc > r_exact - 0.03 and r_inc > 0.9
 
 
-def test_incremental_builder_against_the_reference_builder(tmp_path):
-    """Same points, same levels' distribution, same M / efConstruction: the graph from the GPU insertion builder and the graph
-    from the reference's own HNSW::add_with_locks (compiled, oracle/_ref), both searched with the product's stored-vector
-    traversal at efSearch 64.  Construction is order- and thread-dependent in the reference too, so the comparison is on
-    what the graph is for: recall, and the work a search does on it."""
-    from oracle.binding import Reference, export_to_csr, have_reference
+def builder_points(n, d):
+    x = clustered(n, d, 1000, 5)
+    q = x[:1000] + 0.05 * np.random.default_rng(6).normal(size=(1000, d)).astype(np.float32)
+    return x, q / np.linalg.norm(q, axis=1, keepdims=True)
 
-    if not have_reference():
-        pytest.skip("compiled reference not present")
+
+def reference_builder_recall(n, d, M, efc):
+    """recall@10 at efSearch 64 of the graph that the reference's own HNSW::add_with_locks (compiled, oracle/_ref) builds over
+    builder_points(n, d), searched with the C restatement of the traversal (ids bit-identical to the product's stored-vector
+    search, see test_gpu_search.py), and the graph's links per node."""
+    from oracle.binding import Oracle, Reference, export_to_csr
+
+    x, q = builder_points(n, d)
+    ref = Reference(x.shape[1], M, True)
+    ref.build(x, ef_construction=efc, nthreads=32)
+    g = export_to_csr(ref.export())
+    _, I, _, _ = Oracle(g, x).search(q, 10, ef=64, nthreads=32)
+    gt = np.argsort(-(q @ x.T), axis=1)[:, :10]
+    return float(np.mean([len(set(a.tolist()) & set(b.tolist())) / 10 for a, b in zip(I, gt)])), g.neighbors.size / len(x)
+
+
+def test_incremental_builder_against_the_reference_builder(tmp_path, reference):
+    """Same points, same levels' distribution, same M / efConstruction: the graph from the GPU insertion builder, searched
+    with the product's stored-vector traversal at efSearch 64, and the graph from the reference's own HNSW::add_with_locks
+    (its recall replayed from tests/golden/reference_replay/, see reference_builder_recall).  Construction is order- and
+    thread-dependent in the reference too, so the comparison is on what the graph is for: recall, and the work a search
+    does on it."""
     from leann_b200.graph_build import build_hnsw_graph_incremental
 
     n, d, M, efc = 100_000, 64, 16, 100
-    x = clustered(n, d, 1000, 5)
-    q = x[:1000] + 0.05 * np.random.default_rng(6).normal(size=(1000, d)).astype(np.float32)
-    q /= np.linalg.norm(q, axis=1, keepdims=True)
+    x, q = builder_points(n, d)
     gt = torch.topk(torch.from_numpy(q).cuda() @ torch.from_numpy(x).cuda().T, 10, dim=1).indices.cpu().numpy()
-    ref = Reference(d, M, True)
-    ref.build(x, ef_construction=efc, nthreads=32)
-    g_ref = export_to_csr(ref.export())
+    r_ref, links_ref = reference.proxy(reference_builder_recall, n, d, M, efc)
     g_inc = build_hnsw_graph_incremental(x, M=M, metric="mips", device="cuda", ef_construction=efc)
-    r_ref = _recall_with_product_search(g_ref, x, q, gt, tmp_path, "ref")
     r_inc = _recall_with_product_search(g_inc, x, q, gt, tmp_path, "inc")
-    print(f"recall@10 ef=64: reference builder {r_ref:.3f} ({g_ref.neighbors.size / n:.1f} links/node), "
+    print(f"recall@10 ef=64: reference builder {r_ref:.3f} ({links_ref:.1f} links/node), "
           f"GPU insertion builder {r_inc:.3f} ({g_inc.neighbors.size / n:.1f} links/node)")
     assert r_inc > r_ref - 0.02

@@ -1,12 +1,14 @@
 """The CPU oracle (oracle/hnsw_oracle.c) against the fixtures generated FROM the compiled
-reference (tests/golden/make_golden.py) and, where the prebuilt reference library is present,
-against the reference itself on fresh random inputs."""
+reference (tests/golden/make_golden.py) and against the reference itself on fresh random inputs
+(its outputs replayed from tests/golden/reference_replay/, see helpers.ReferenceReplay)."""
+import ctypes as C
+
 import numpy as np
 import pytest
 
-from helpers import GOLDEN_CASES, golden_key
+from helpers import GOLDEN_CASES, golden_key, reference  # noqa: F401  (reference: fixture)
 from leann_b200.csr import read_compact_index
-from oracle.binding import Oracle, Reference, have_reference
+from oracle.binding import HERE, Oracle, Reference
 
 
 @pytest.fixture(scope="module")
@@ -34,14 +36,13 @@ def test_golden_has_distance_ties(fx):
     assert any(len(np.unique(row)) < len(row) for row in D)
 
 
-@pytest.mark.skipif(not have_reference(), reason="oracle/_ref not built (only possible in the dev container)")
 @pytest.mark.parametrize("metric_ip", [True, False])
-def test_oracle_vs_compiled_reference_random(metric_ip):
+def test_oracle_vs_compiled_reference_random(metric_ip, reference):
     rng = np.random.default_rng(7)
     n, d = 3000, 48
     x = rng.standard_normal((n, d)).astype(np.float32)
     q = rng.standard_normal((40, d)).astype(np.float32)
-    R = Reference(d, M=8, metric_ip=metric_ip)
+    R = reference.proxy(Reference, d, M=8, metric_ip=metric_ip)
     R.build(x, ef_construction=40, nthreads=1)
     from oracle.binding import export_to_csr
     g = export_to_csr(R.export())
@@ -53,9 +54,8 @@ def test_oracle_vs_compiled_reference_random(metric_ip):
             assert np.array_equal(u, v)
 
 
-@pytest.mark.skipif(not have_reference(), reason="oracle/_ref not built (only possible in the dev container)")
 @pytest.mark.parametrize("seed", range(10))
-def test_oracle_vs_compiled_reference_fuzz(seed):
+def test_oracle_vs_compiled_reference_fuzz(seed, reference):
     """Randomised shapes and search parameters, on purpose degenerate: integer-valued coordinates (many exactly equal
     distances -> every tie-break of the heaps, the beam and the result handler matters), duplicate vectors, k above and below
     efSearch, more results requested than nodes reachable, beam / batch modes, both metrics, the relative-distance stop rule on
@@ -69,7 +69,7 @@ def test_oracle_vs_compiled_reference_fuzz(seed):
     x = rng.integers(-3, 4, (n, d)).astype(np.float32)
     x[rng.integers(0, n, n // 10 + 1)] = x[0]                      # exact duplicates of one vector
     q = np.concatenate([rng.integers(-3, 4, (12, d)), x[:4]]).astype(np.float32)   # some queries ARE data points
-    R = Reference(d, M=M, metric_ip=metric_ip)
+    R = reference.proxy(Reference, d, M=M, metric_ip=metric_ip)
     R.build(x, ef_construction=int(rng.choice([16, 40])), nthreads=1)
     O = Oracle(export_to_csr(R.export()), x)
     for _ in range(5):
@@ -84,36 +84,59 @@ def test_oracle_vs_compiled_reference_fuzz(seed):
             assert np.array_equal(u, v), (name, dict(n=n, d=d, M=M, ip=metric_ip, ef=ef, beam=beam, batch=batch, cr=cr, k=k))
 
 
-@pytest.mark.skipif(not have_reference(), reason="oracle/_ref not built")
-def test_minimax_heap_vs_reference():
+class MinimaxHeap:
+    """The MinimaxHeap entry points of the compiled reference (which="ref": ref_mmh_* of oracle/_ref/libleann_ref.so) or
+    of the C restatement (which="oracle": lbo_mmh_* of oracle/liboracle.so)."""
+
+    def __init__(self, which):
+        lib, prefix = {"ref": (HERE / "_ref" / "libleann_ref.so", "ref_mmh_"), "oracle": (HERE / "liboracle.so", "lbo_mmh_")}[which]
+        lib = C.CDLL(str(lib))
+        self.f = {f: getattr(lib, prefix + f) for f in ("new", "push", "pop_min", "count_below", "size", "free")}
+        self.f["new"].restype = C.c_void_p
+        for f, a in {"push": [C.c_void_p, C.c_int, C.c_float], "pop_min": [C.c_void_p, C.POINTER(C.c_float)],
+                     "count_below": [C.c_void_p, C.c_float], "size": [C.c_void_p], "free": [C.c_void_p]}.items():
+            self.f[f].argtypes = a
+
+    def new(self, cap):
+        return self.f["new"](cap)
+
+    def push(self, h, i, v):
+        self.f["push"](h, i, v)
+
+    def pop_min(self, h):
+        v = C.c_float()
+        return self.f["pop_min"](h, C.byref(v)), v.value
+
+    def count_below(self, h, t):
+        return self.f["count_below"](h, t)
+
+    def size(self, h):
+        return self.f["size"](h)
+
+    def free(self, h):
+        self.f["free"](h)
+
+
+def test_minimax_heap_vs_reference(reference):
     """Random push / pop_min / count_below traces incl. equal and infinite distances
     (shape of faiss/tests/test_hnsw.cpp:20-195)."""
-    import ctypes as C
-    from oracle.binding import HERE
-    ref = C.CDLL(str(HERE / "_ref" / "libleann_ref.so"))
-    ora = C.CDLL(str(HERE / "liboracle.so"))
-    for lib, p in ((ref, "ref_mmh_"), (ora, "lbo_mmh_")):
-        getattr(lib, p + "new").restype = C.c_void_p
-        for f in ("push", "pop_min", "count_below", "size", "free"):
-            getattr(lib, p + f).argtypes = {"push": [C.c_void_p, C.c_int, C.c_float], "pop_min": [C.c_void_p, C.POINTER(C.c_float)],
-                                            "count_below": [C.c_void_p, C.c_float], "size": [C.c_void_p], "free": [C.c_void_p]}[f]
+    ref = reference.proxy(MinimaxHeap, "ref")
+    ora = MinimaxHeap("oracle")
     rng = np.random.default_rng(3)
     for trial in range(30):
         cap = int(rng.integers(1, 40))
-        hr, ho = ref.ref_mmh_new(cap), ora.lbo_mmh_new(cap)
+        hr, ho = ref.new(cap), ora.new(cap)
         vals = np.concatenate([rng.integers(0, 8, 200).astype(np.float32), [np.inf] * 5])
         for step in range(400):
             op = rng.random()
             if op < 0.6:
                 i, v = int(rng.integers(0, 1000)), float(rng.choice(vals))
-                ref.ref_mmh_push(hr, i, v); ora.lbo_mmh_push(ho, i, v)
+                ref.push(hr, i, v); ora.push(ho, i, v)
             elif op < 0.85:
-                if ref.ref_mmh_size(hr) > 0:
-                    a, b = C.c_float(), C.c_float()
-                    assert ref.ref_mmh_pop_min(hr, C.byref(a)) == ora.lbo_mmh_pop_min(ho, C.byref(b))
-                    assert a.value == b.value
+                if ref.size(hr) > 0:
+                    assert ref.pop_min(hr) == ora.pop_min(ho)
             else:
                 t = float(rng.choice(vals))
-                assert ref.ref_mmh_count_below(hr, t) == ora.lbo_mmh_count_below(ho, t)
-            assert ref.ref_mmh_size(hr) == ora.lbo_mmh_size(ho)
-        ref.ref_mmh_free(hr); ora.lbo_mmh_free(ho)
+                assert ref.count_below(hr, t) == ora.count_below(ho, t)
+            assert ref.size(hr) == ora.size(ho)
+        ref.free(hr); ora.free(ho)

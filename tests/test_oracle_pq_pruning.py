@@ -1,15 +1,15 @@
 """PQ-guided pruning of the HNSW search (SURVEY 8f row 3; faiss/impl/HNSW_search.cpp:442-465, 645-750 + impl/pq.cpp):
 the C restatement (oracle/hnsw_oracle.c) against the reference's own compiled code (oracle/_ref/libleann_ref.so with
-HNSW::load_pq_pruning_data reading DiskANN-format PQ files) — ids, distances, ndis, nhops identical for the three
-selection strategies (global / local / proportional), beams, batch mode and both metrics."""
+HNSW::load_pq_pruning_data reading DiskANN-format PQ files; its outputs replayed from tests/golden/reference_replay/) — ids,
+distances, ndis, nhops identical for the three selection strategies (global / local / proportional), beams, batch mode and
+both metrics."""
 import numpy as np
 import pytest
 
 from leann_b200.graph_build import build_hnsw_graph
 from leann_b200.vamana_build import build_diskann_index
-from oracle.binding import Oracle, Reference, have_reference
-
-needs_ref = pytest.mark.skipif(not have_reference(), reason="compiled reference not present (GPU box)")
+from helpers import reference  # noqa: F401  (fixture)
+from oracle.binding import Oracle, Reference
 
 PRUNE_CASES = [  # (prune_ratio, local_prune, send_ratio, ef, beam, batch, check_rel, k)
     (0.5, False, 0.0, 32, 1, 0, True, 10), (0.8, False, 0.0, 64, 1, 0, True, 10), (0.3, False, 0.0, 24, 4, 0, True, 5),
@@ -33,11 +33,10 @@ def make_world(tmp_path, metric, n=4000, d=32, n_chunks=16, seed=0):
     return dict(x=x, q=q, g=g, pq=pq, codes=codes, prefix=prefix)
 
 
-@needs_ref
 @pytest.mark.parametrize("metric", ["mips", "l2"])
-def test_pq_pruning_restatement_matches_the_compiled_reference(tmp_path, metric):
+def test_pq_pruning_restatement_matches_the_compiled_reference(tmp_path, metric, reference):
     W = make_world(tmp_path, metric)
-    ref = Reference.from_csr(W["g"], W["x"], M=8)
+    ref = reference.proxy(Reference.from_csr, W["g"], W["x"], M=8)
     ref.load_pq(W["prefix"] + "_pq_pivots.bin", W["prefix"] + "_pq_compressed.bin")
     o = Oracle(W["g"], W["x"])
     o.set_pq(W["pq"], W["codes"])
@@ -55,13 +54,12 @@ def test_pq_pruning_restatement_matches_the_compiled_reference(tmp_path, metric)
         assert np.array_equal(u, v)
 
 
-@needs_ref
-def test_pq_lookup_table_matches_the_reference_bit_for_bit(tmp_path):
+def test_pq_lookup_table_matches_the_reference_bit_for_bit(tmp_path, reference):
     """lbo_pq_lut / lbo_pq_dist against a search that is driven entirely by the table: with local pruning at ratio ~0 nothing
     is selected unless ... instead compare through ndis of many ratios: covered above; here: odd chunk widths and a PQ
     whose dimension is not d + 1 aligned."""
     W = make_world(tmp_path, "mips", n=1500, d=20, n_chunks=7, seed=3)
-    ref = Reference.from_csr(W["g"], W["x"], M=8)
+    ref = reference.proxy(Reference.from_csr, W["g"], W["x"], M=8)
     ref.load_pq(W["prefix"] + "_pq_pivots.bin", W["prefix"] + "_pq_compressed.bin")
     o = Oracle(W["g"], W["x"])
     o.set_pq(W["pq"], W["codes"])

@@ -1,5 +1,7 @@
 """CPU suite for the DiskANN/Vamana row: file formats, and the C restatement's primitives pinned against the
-reference's own code (oracle/_ref/libleann_ref_diskann.so = DiskANN's neighbor.h + pq.cpp compiled here)."""
+reference's own code (oracle/_ref/libleann_ref_diskann.so = DiskANN's neighbor.h + pq.cpp, and
+oracle/_ref/libleann_ref_diskann_flash.so = its PQFlashIndex search loop; their outputs replayed from
+tests/golden/reference_replay/, see helpers.ReferenceReplay)."""
 from __future__ import annotations
 
 import numpy as np
@@ -7,10 +9,9 @@ import pytest
 
 from leann_b200 import diskann_format as dfmt
 from leann_b200.vamana_build import build_diskann_index, build_vamana_graph
-from oracle.vamana_binding import (DiskannFlash, DiskannPrimitives, OracleQueue, VamanaOracle, have_diskann_flash,
-                                   have_diskann_reference)
+from helpers import reference  # noqa: F401  (fixture)
+from oracle.vamana_binding import DiskannFlash, DiskannPrimitives, OracleQueue, VamanaOracle, have_diskann_flash
 
-needs_ref = pytest.mark.skipif(not have_diskann_reference(), reason="compiled DiskANN primitives not present")
 needs_flash = pytest.mark.skipif(not have_diskann_flash(), reason="compiled PQFlashIndex (oracle/_ref/libleann_ref_diskann_flash.so) not present")
 
 
@@ -64,10 +65,9 @@ def test_prepare_base_matches_the_searchers_preprocessing(small_index):
     assert abs(np.linalg.norm(s["coords"], axis=1).max() - 1.0) < 1e-5
 
 
-@needs_ref
-def test_queue_restatement_matches_reference_queue():
+def test_queue_restatement_matches_reference_queue(reference):
     """Random insert / closest_unexpanded streams incl. distance ties, duplicate ids and a full queue."""
-    ref = DiskannPrimitives()
+    ref = reference.proxy(DiskannPrimitives)
     rng = np.random.default_rng(5)
     for cap in (1, 4, 17, 64):
         a, b = ref.queue(cap), OracleQueue(cap)
@@ -84,14 +84,13 @@ def test_queue_restatement_matches_reference_queue():
         assert a.items() == b.items()
 
 
-@needs_ref
 @pytest.mark.parametrize("metric", ["mips", "l2"])
-def test_pq_restatement_matches_reference_pq_bit_for_bit(tmp_path, metric):
+def test_pq_restatement_matches_reference_pq_bit_for_bit(tmp_path, metric, reference):
     emb = unit_rows(900, 41, 3)  # 41 (+1) dims over 9 chunks: uneven chunk widths
     prefix, g, coords, pq, codes, max_norm = build_diskann_index(tmp_path, "p", emb, metric=metric, R=8, n_chunks=9, device="cpu")
-    ref = DiskannPrimitives()
+    ref = reference.proxy(DiskannPrimitives)
     table = ref.pq_load(prefix + "_pq_pivots.bin", pq.n_chunks)
-    assert ref.lib.dref_pq_num_chunks(table) == pq.n_chunks
+    assert ref.pq_num_chunks(table) == pq.n_chunks
     o = VamanaOracle(g, pq, codes, metric, max_norm)
     rng = np.random.default_rng(9)
     for _ in range(5):
@@ -136,13 +135,12 @@ def test_oracle_search_finds_true_neighbours(tmp_path, metric):
     assert info["n_full"].min() >= 10 and (info["n_ios"] == info["n_full"]).all()
 
 
-@needs_ref
 @pytest.mark.parametrize("metric", ["mips", "l2"])
-def test_reference_pq_reads_the_committed_fixture(golden_dir, metric):
+def test_reference_pq_reads_the_committed_fixture(golden_dir, metric, reference):
     """The reference's own load_pq_centroid_bin / populate_chunk_distances / pq_dist_lookup on the committed files."""
     from helpers import load_vamana_golden
     G = load_vamana_golden(golden_dir, metric)
-    ref = DiskannPrimitives()
+    ref = reference.proxy(DiskannPrimitives)
     table = ref.pq_load(G["prefix"] + "_pq_pivots.bin", G["pq"].n_chunks)
     o = VamanaOracle(G["g"], G["pq"], G["codes"], metric, G["max_norm"])
     q = np.zeros(G["pq"].ndims, np.float32)
@@ -174,11 +172,11 @@ def _beam_search_with_reference_primitives(ref, table, G, q, L, beam, k, io_limi
     2419-2612, 2761, 2861-2883; L2 metric, skip_search_reorder) driving the REFERENCE's compiled queue and PQ table, so the
     only non-reference code involved is this loop."""
     g, codes, n_chunks = G["g"], G["codes"], G["pq"].n_chunks
-    _, lut = ref.lut(table, q, n_chunks)                      # preprocess_query + populate_chunk_distances
+    qt = ref.query_table(table, q, n_chunks)                  # preprocess_query + populate_chunk_distances
     retset = ref.queue(L)
     visited = set()
     med = g.medoid
-    retset.insert(med, float(ref.pq_dists(lut, [med], codes)[0]))
+    retset.insert(med, float(qt.dists([med], codes)[0]))
     visited.add(med)
     full, cmps, hops, ios = [], 0, 0, 0
     while retset.has_unexpanded() and ios < io_limit:
@@ -192,7 +190,7 @@ def _beam_search_with_reference_primitives(ref, table, G, q, L, beam, k, io_limi
             full.append((d, node))
             nb = g.nbrs[node]
             nb = nb[nb >= 0]
-            dists = ref.pq_dists(lut, nb, codes)
+            dists = qt.dists(nb, codes)
             for m, i in enumerate(nb.tolist()):
                 if i not in visited:
                     visited.add(i)
@@ -209,11 +207,10 @@ def _beam_search_with_reference_primitives(ref, table, G, q, L, beam, k, io_limi
     return np.array(ids), ds, [i for _, i in full], cmps, hops
 
 
-@needs_ref
-def test_search_loop_agrees_with_a_second_transcription_over_reference_primitives(golden_dir):
+def test_search_loop_agrees_with_a_second_transcription_over_reference_primitives(golden_dir, reference):
     from helpers import load_vamana_golden
     G = load_vamana_golden(golden_dir, "l2")
-    ref = DiskannPrimitives()
+    ref = reference.proxy(DiskannPrimitives)
     table = ref.pq_load(G["prefix"] + "_pq_pivots.bin", G["pq"].n_chunks)
     o = VamanaOracle(G["g"], G["pq"], G["codes"], "l2", 0.0)
     for L, beam, k, io_limit in [(64, 1, 10, 2 ** 32 - 1), (16, 4, 10, 2 ** 32 - 1), (8, 3, 20, 2 ** 32 - 1), (32, 2, 5, 9)]:
@@ -226,13 +223,12 @@ def test_search_loop_agrees_with_a_second_transcription_over_reference_primitive
             assert np.array_equal(I[qi], ids) and np.array_equal(D[qi], ds)
 
 
-@needs_ref
-def test_search_loop_second_transcription_mips_with_query_normalisation(golden_dir):
+def test_search_loop_second_transcription_mips_with_query_normalisation(golden_dir, reference):
     """Same cross-check for the MIPS index: the query is normalised / extended by the oracle's vo_prepare_query, everything
     after that (centring, table, queue, distances) is the reference's compiled code."""
     from helpers import load_vamana_golden
     G = load_vamana_golden(golden_dir, "mips")
-    ref = DiskannPrimitives()
+    ref = reference.proxy(DiskannPrimitives)
     table = ref.pq_load(G["prefix"] + "_pq_pivots.bin", G["pq"].n_chunks)
     o = VamanaOracle(G["g"], G["pq"], G["codes"], "mips", G["max_norm"])
     for L, beam, k in [(64, 1, 10), (16, 4, 10)]:
@@ -312,9 +308,8 @@ def test_compiled_reference_reproduces_its_committed_outputs(golden_dir, metric)
                 assert np.array_equal(st["n_cmps"], G["exp"][key + "_refcmps"]) and np.array_equal(st["n_hops"], G["exp"][key + "_refhops"])
 
 
-@needs_flash
 @pytest.mark.parametrize("metric,R,n_chunks,dim", [("l2", 16, 12, 48), ("mips", 24, 10, 40), ("cosine", 12, 8, 32), ("mips", 32, 17, 51)])
-def test_compiled_reference_search_loop_pins_the_oracle_on_fresh_indexes(tmp_path, metric, R, n_chunks, dim):
+def test_compiled_reference_search_loop_pins_the_oracle_on_fresh_indexes(tmp_path, metric, R, n_chunks, dim, reference):
     """Fresh random indexes (both file layouts), beam widths 1..8, tiny and huge L, io_limit: the restatement follows the
     compiled reference expansion for expansion (hops, I/Os, comparison counts) and returns the same ids."""
     emb = unit_rows(2500, dim, 11 + R)
@@ -325,7 +320,7 @@ def test_compiled_reference_search_loop_pins_the_oracle_on_fresh_indexes(tmp_pat
     q = unit_rows(16, dim, 99)
     o = VamanaOracle(g, pq, codes, metric, max_norm)
     for part in ("", prefix):
-        ref = DiskannFlash(prefix, metric, partition_prefix=part)
+        ref = reference.proxy(DiskannFlash, prefix, metric, partition_prefix=part)
         ref.set_embeddings(emb)
         for L, beam, k, io_limit in ((64, 1, 10, 2 ** 32 - 1), (10, 2, 10, 2 ** 32 - 1), (150, 4, 20, 2 ** 32 - 1), (64, 8, 5, 2 ** 32 - 1),
                                      (64, 2, 10, 7), (32, 1, 3, 1)):

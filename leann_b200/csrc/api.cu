@@ -298,8 +298,7 @@ int next_pow2(int v) {
 
 // embed, work list, pool + per layer: 4 GEMMs, attention, and 2 LayerNorm kernels unless they ride in the GEMM epilogues
 int encoder_kernels_per_pass(const Encoder& e) {
-    const bool fused_ln = e.cfg.hidden == 2 * gemm_block_n() && !(getenv("LB2_FUSED_LN") && atoi(getenv("LB2_FUSED_LN")) == 0);
-    return 3 + e.cfg.layers * (fused_ln ? 5 : 7);
+    return 3 + e.cfg.layers * (encoder_fuses_ln(e.cfg) ? 5 : 7);
 }
 
 int search_impl(lb2_index* x, int64_t nq, const float* d_q, int64_t k, float* d_D, int64_t* d_I,

@@ -22,8 +22,6 @@
 #include <cuda_fp16.h>
 
 #include "common.cuh"
-#include <cstdlib>
-
 #include "ptx.cuh"
 
 namespace lb2 {
@@ -35,14 +33,12 @@ constexpr int ATC_TM = 128;    // query rows per item
 constexpr int ATC_MAXL = 256;  // keys per passage (TMEM columns of S)
 constexpr int ATC_BOX = 64;    // rows per TMA box
 constexpr int ATC_THREADS = 192;     // 4 softmax warps + TMA + MMA
-constexpr int ATC_THREADS8 = 320;    // 8 softmax warps (two per row quarter, each half of the key chunks) + TMA + MMA
 constexpr int ATC_QK_BYTES = ATC_MAXL * 128;
 constexpr int ATC_V_BYTES = ATC_MAXL * 64;
 constexpr int ATC_STAGE_BYTES = ATC_QK_BYTES + ATC_V_BYTES;
 constexpr int ATC_STAGES = 2;
 constexpr int ATC_BAR_OFFSET = ATC_STAGES * ATC_STAGE_BYTES;
-constexpr int ATC_X_OFFSET = ATC_BAR_OFFSET + 256;          // 8-warp softmax: row maxima / partial sums exchanged between the two warps of a row
-constexpr int ATC_SMEM = ATC_X_OFFSET + 2 * 2 * 2 * 128 * 4 + 1024;
+constexpr int ATC_SMEM = ATC_BAR_OFFSET + 256 + 1024;
 constexpr int ATC_TMEM_COLS = 256;
 constexpr int ATC_O_COL0 = 192;  // two O accumulators of 32 columns at the top of the allocation
 constexpr int ATC_LONG = 192;    // an item whose S needs more columns than this overlaps them ("long" item)
@@ -57,33 +53,22 @@ __device__ __forceinline__ uint32_t pack2(float a, float b) {
     return *reinterpret_cast<const uint32_t*>(&h);
 }
 
-// work list: one descriptor per (passage, 128-row query block): {first packed row of the passage, length, query window, passage}.
-// One 16-byte load per work item in the kernel (no dependent items -> seq_len -> seq_start chain); a passage's blocks are adjacent.
-// query window z = q0 | lo << 16: the item's 128 MMA rows are the passage's rows [q0, q0 + 128); rows in [lo, L) are its
-// output.  First block: q0 = lo = 0.  Second block (rows 128 .. L-1, usually only one or two warps' worth): q0 = lo = 128,
-// or — LB2_ATTN_ROTATE=1, an experiment kept as a switch — q0 = 128 - 32 * rot, which puts the tail rot row quarters up
-// (the A operand is the same (q | k) tile, only the descriptor start moves by rot * 4 KB; the warps below lo idle).
-// Why: softmax warp w lives on SM sub-partition w, and with every tail in quarter 0 sub-partition 0 carries 1.31x the mean
-// MUFU load on the bench corpus' length mix (N(128, 48)), sub-partition 3 0.72x; the tables below bring max / mean to 1.01
-// (scripts/attn_rotation_model.py).  Measured (profiles/r02e_attention_rotation_ab.log): bit-identical outputs and NO
-// change in time (0.786 vs 0.788 ms) — the kernel is bound by the per-item chain S -> softmax -> P.V of a CTA (a tail item
-// costs a full item whatever its warps do), not by MUFU throughput per sub-partition.  Default off.
-__constant__ uint8_t ATC_ROT1[8] = {3, 3, 3, 3, 3, 3, 0, 1};  // tail of <= 32 rows
-__constant__ uint8_t ATC_ROT2[8] = {2, 2, 2, 2, 2, 0, 0, 0};  // tail of <= 64 rows (<= 96 and more: no rotation)
+// work list: one descriptor per (passage, 128-row query block): {first packed row of the passage, length, first query row
+// q0, passage}.  One 16-byte load per work item in the kernel (no dependent items -> seq_len -> seq_start chain); a passage's
+// blocks are adjacent.  The item's 128 MMA rows are the passage's rows [q0, q0 + 128); rows in [q0, L) are its output.
+// First block: q0 = 0.  Second block (rows 128 .. L-1, usually only one or two warps' worth): q0 = 128, so a tail always
+// sits in row quarter 0.  Spreading tails over the row quarters evens out the MUFU load of the SM sub-partitions but leaves
+// the time unchanged (profiles/r02e_attention_rotation_ab.log): the kernel is bound by the per-item chain S -> softmax ->
+// P.V of a CTA (a tail item costs a full item whatever its warps do), not by MUFU throughput per sub-partition.
 __global__ void attention_tc_items_kernel(const int32_t* __restrict__ seq_start, const int32_t* __restrict__ seq_len, int n_seq,
-                                          int row_base, int4* __restrict__ desc, int* __restrict__ count, int rotate) {
+                                          int row_base, int4* __restrict__ desc, int* __restrict__ count) {
     const int s = blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= n_seq) return;
     const int L = seq_len[s];
     const int nb = (L + ATC_TM - 1) / ATC_TM;
     const int base = atomicAdd(count, nb);
     desc[base] = make_int4(seq_start[s] - row_base, L, 0, s);
-    if (nb > 1) {
-        const int wt = (L - ATC_TM + 31) >> 5;  // warps the tail occupies
-        const unsigned hsh = (static_cast<unsigned>(s) * 2654435761u) >> 13;
-        const int rot = !rotate ? 0 : wt == 1 ? ATC_ROT1[hsh & 7] : wt == 2 ? ATC_ROT2[hsh & 7] : 0;
-        desc[base + 1] = make_int4(seq_start[s] - row_base, L, (ATC_TM - 32 * rot) | (ATC_TM << 16), s);
-    }
+    if (nb > 1) desc[base + 1] = make_int4(seq_start[s] - row_base, L, ATC_TM, s);
 }
 
 // Pipeline of one CTA over its items i = 0, 1, ... (two CTAs per SM interleave):
@@ -92,11 +77,10 @@ __global__ void attention_tc_items_kernel(const int32_t* __restrict__ seq_start,
 //   softmax warps: for i: wait S(i) -> softmax -> P(i) | read O(i - 1) out while P.V(i) and S(i + 1) execute
 // so the chain per item is softmax -> P.V + S, and the O read-out, the TMA loads and the other CTA's softmax fill the gaps.
 // A long item (S wider than 192 columns) would overwrite the O accumulators: both sides drain the pending read-outs first.
-template <int SW>
-__global__ void __launch_bounds__(SW * 32 + 64, 2)
+__global__ void __launch_bounds__(ATC_THREADS, 2)
 attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qk, const __grid_constant__ CUtensorMap tmap_v,
                     const int4* __restrict__ desc, const int* __restrict__ n_items, int heads, int hidden,
-                    __half* __restrict__ ctx, unsigned wait_ns, int skip_empty) {
+                    __half* __restrict__ ctx) {
     extern __shared__ uint8_t att_smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(att_smem_raw) + 1023) & ~uintptr_t(1023));
     uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + ATC_BAR_OFFSET);
@@ -111,7 +95,7 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qk, const __grid_co
     const int total = *n_items * heads;
     const int n_it = total > static_cast<int>(blockIdx.x) ? (total - static_cast<int>(blockIdx.x) + static_cast<int>(gridDim.x) - 1) / static_cast<int>(gridDim.x) : 0;
 
-    if (warp == SW && lane == 0) {
+    if (warp == 4 && lane == 0) {
         ptx::prefetch_tmap(&tmap_qk);
         ptx::prefetch_tmap(&tmap_v);
         for (int i = 0; i < ATC_STAGES; i++) {
@@ -119,14 +103,14 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qk, const __grid_co
             ptx::mbar_init(&empty_bar[i], 1);
         }
         ptx::mbar_init(s_ready, 1);
-        ptx::mbar_init(p_ready, SW);
+        ptx::mbar_init(p_ready, 4);
         for (int i = 0; i < 2; i++) {
             ptx::mbar_init(&o_ready[i], 1);
-            ptx::mbar_init(&o_free[i], SW);
+            ptx::mbar_init(&o_free[i], 4);
         }
         ptx::fence_barrier_init();
     }
-    if (warp == SW + 1) {
+    if (warp == 5) {
         ptx::tmem_alloc(tmem_ptr, ATC_TMEM_COLS);
         ptx::tmem_relinquish();
     }
@@ -135,7 +119,7 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qk, const __grid_co
     ptx::tc_fence_after();
     const uint32_t tmem_base = *tmem_ptr;
 
-    if (warp == SW) {
+    if (warp == 4) {
         // ===== TMA producer, whole warp + one elected issuer (the descriptor of the next item is fetched while this one's
         // loads are issued)
         int4 cur = n_it > 0 ? __ldg(&desc[blockIdx.x / heads]) : make_int4(0, 0, 0, 0);
@@ -148,7 +132,7 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qk, const __grid_co
             const int L = cur.y;
             const int row0 = cur.x;
             const int nbox = (L + ATC_BOX - 1) / ATC_BOX;
-            ptx::mbar_wait_ns(&empty_bar[stage], ph ^ 1, wait_ns);
+            ptx::mbar_wait(&empty_bar[stage], ph ^ 1);
             uint8_t* qk = smem + stage * ATC_STAGE_BYTES;
             uint8_t* v = qk + ATC_QK_BYTES;
             if (ptx::elect_one()) {
@@ -161,7 +145,7 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qk, const __grid_co
             __syncwarp();
             cur = nxt;
         }
-    } else if (warp == SW + 1) {
+    } else if (warp == 5) {
         if (n_it > 0) {
             // ===== MMA issuer: the whole warp runs the loop, one elected lane issues (warp-uniform control flow keeps the
             // descriptors in uniform registers; under `if (lane == 0)` every tcgen05.mma sat in an ELECT / R2UR.BROADCAST
@@ -169,7 +153,7 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qk, const __grid_co
             auto issue_s = [&](int it, const int4& d) {
                 const int Lp = (d.y + 15) & ~15;
                 const uint32_t qk = ptx::smem_u32(smem + (it & 1) * ATC_STAGE_BYTES);
-                const uint64_t a_desc = ptx::make_sw128_kmajor_desc(qk + (d.z & 0xffff) * 128);  // query window start q0 (a multiple of 32 rows = 4 KB)
+                const uint64_t a_desc = ptx::make_sw128_kmajor_desc(qk + d.z * 128);  // first query row q0 (0 or 128)
                 const uint64_t b_desc = ptx::make_sw128_kmajor_desc(qk) + 4;  // the k half of the (q | k) rows: +64 B
                 const uint32_t idesc_s = ptx::make_idesc_f16(ATC_TM, Lp);
                 if (ptx::elect_one()) {
@@ -182,15 +166,15 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qk, const __grid_co
             };
             int4 cur = __ldg(&desc[blockIdx.x / heads]);
             int4 nxt = n_it > 1 ? __ldg(&desc[(blockIdx.x + gridDim.x) / heads]) : cur;
-            ptx::mbar_wait_ns(&full_bar[0], 0, wait_ns);
+            ptx::mbar_wait(&full_bar[0], 0);
             ptx::tc_fence_after();
             issue_s(0, cur);
             for (int it = 0; it < n_it; it++) {
                 const int stage = it & 1, b = it & 1;
                 const int Lp = (cur.y + 15) & ~15;
                 const int4 nn = it + 2 < n_it ? __ldg(&desc[(blockIdx.x + (it + 2) * gridDim.x) / heads]) : nxt;
-                ptx::mbar_wait_ns(p_ready, it & 1, wait_ns);
-                ptx::mbar_wait_ns(&o_free[b], ((it >> 1) & 1) ^ 1, wait_ns);  // the previous user of this O accumulator has been read out
+                ptx::mbar_wait(p_ready, it & 1);
+                ptx::mbar_wait(&o_free[b], ((it >> 1) & 1) ^ 1);  // the previous user of this O accumulator has been read out
                 ptx::tc_fence_after();
                 const uint32_t vb = ptx::smem_u32(smem + stage * ATC_STAGE_BYTES) + ATC_QK_BYTES;
                 const uint32_t idesc_o = ptx::make_idesc_f16(ATC_TM, ATC_HD) | ptx::IDESC_B_MN_MAJOR;
@@ -203,10 +187,10 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qk, const __grid_co
                 }
                 __syncwarp();
                 if (it + 1 < n_it) {
-                    ptx::mbar_wait_ns(&full_bar[(it + 1) & 1], ((it + 1) >> 1) & 1, wait_ns);
+                    ptx::mbar_wait(&full_bar[(it + 1) & 1], ((it + 1) >> 1) & 1);
                     if (((nxt.y + 15) & ~15) > ATC_LONG) {  // S(it + 1) covers the O accumulators: O(it) and O(it - 1) must be out
-                        ptx::mbar_wait_ns(&o_free[b], (it >> 1) & 1, wait_ns);
-                        if (it >= 1) ptx::mbar_wait_ns(&o_free[b ^ 1], ((it - 1) >> 1) & 1, wait_ns);
+                        ptx::mbar_wait(&o_free[b], (it >> 1) & 1);
+                        if (it >= 1) ptx::mbar_wait(&o_free[b ^ 1], ((it - 1) >> 1) & 1);
                     }
                     ptx::tc_fence_after();
                     issue_s(it + 1, nxt);
@@ -215,7 +199,7 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qk, const __grid_co
                 nxt = nn;
             }
         }
-    } else if (SW == 4) {
+    } else {
         // ===== softmax + output: thread = query row
         const float scale_log2 = rsqrtf(static_cast<float>(ATC_HD)) * 1.4426950408889634f;
         const uint32_t taddr = tmem_base + (static_cast<uint32_t>(warp * 32) << 16);
@@ -254,13 +238,12 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qk, const __grid_co
             const int w = blockIdx.x + it * gridDim.x;
             const int4 nxt = it + 1 < n_it ? __ldg(&desc[(w + gridDim.x) / heads]) : cur;  // in flight during this item's softmax
             const int h = w % heads;
-            const int q0 = cur.z & 0xffff, lo = cur.z >> 16;
+            const int q0 = cur.z;
             const int L = cur.y;
             const int q = q0 + threadIdx.x;
-            // a warp whose 32 query rows all lie outside [lo, L) (short passages; second query block: rows beyond the passage
-            // and first-block rows under a rotated window) runs zero key chunks: no exponentials, no P rows (its O rows are
-            // never stored) — only the barrier protocol
-            const int nch = (skip_empty && (q0 + warp * 32 >= L || q0 + warp * 32 + 32 <= lo)) ? 0 : (L + 31) >> 5;
+            // a warp whose 32 query rows all lie beyond the passage (short passages; the second query block) runs zero key
+            // chunks: no exponentials, no P rows (its O rows are never stored) — only the barrier protocol
+            const int nch = q0 + warp * 32 >= L ? 0 : (L + 31) >> 5;
             if (((L + 15) & ~15) > ATC_LONG)  // the MMA warp waits for these before it may issue S(it)
                 while (pend < it) readout(pend++);
             ptx::mbar_wait(s_ready, it & 1);
@@ -330,7 +313,7 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qk, const __grid_co
             __syncwarp();
             if (lane == 0) ptx::mbar_arrive(p_ready);
             const float inv = 1.0f / sum;
-            const long long off = (q >= lo && q < L) ? static_cast<long long>(cur.x + q) * hidden + h * ATC_HD : -1;
+            const long long off = q < L ? static_cast<long long>(cur.x + q) * hidden + h * ATC_HD : -1;
             if (it & 1) { inv_sum[1] = inv; out_off[1] = off; } else { inv_sum[0] = inv; out_off[0] = off; }
             while (pend < it) readout(pend++);  // O(it - 1): its P.V was issued long ago; runs while P.V(it) and S(it + 1) execute
             cur = nxt;
@@ -338,137 +321,9 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qk, const __grid_co
         while (pend < n_it) readout(pend++);
     }
 
-    else {
-        // ===== softmax + output with EIGHT warps: warps w and w + 4 share the query rows of TMEM lane quarter w & 3 and split
-        // the 32-key chunks (even / odd).  Twice the warps per SM sub-partition for the exponentials and the tcgen05.ld
-        // latencies (the 4-warp version kept MUFU 33 % busy), half the softmax latency per item.  Costs: the row maximum and
-        // the row sum are combined through shared memory (one 64-thread named barrier per pair), and because P(c) is
-        // written over the columns of S chunk c / 2 — possibly the OTHER warp's — pass 2 runs in rounds of two chunks with a
-        // pair barrier between the reads and the writes of a round.
-        const float scale_log2 = rsqrtf(static_cast<float>(ATC_HD)) * 1.4426950408889634f;
-        const int q4 = warp & 3, hh = warp >> 2;
-        const int row = q4 * 32 + lane;
-        const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q4 * 32) << 16);
-        float* xmax = reinterpret_cast<float*>(smem + ATC_X_OFFSET);  // [item parity][half][row]
-        float* xsum = xmax + 2 * 2 * 128;                              // [item parity][half][row]
-        auto pair_sync = [&]() {  // named barrier 1 + q4 of the two warps that share this row quarter (immediate ids: 5 barriers per CTA)
-            if (q4 == 0) asm volatile("bar.sync 1, 64;" ::: "memory");
-            else if (q4 == 1) asm volatile("bar.sync 2, 64;" ::: "memory");
-            else if (q4 == 2) asm volatile("bar.sync 3, 64;" ::: "memory");
-            else asm volatile("bar.sync 4, 64;" ::: "memory");
-        };
-        long long out_off[2] = {-1, -1};
-        int pend = 0;
-
-        auto readout = [&](int j) {
-            const int b = j & 1;
-            uint32_t o[16];
-            ptx::mbar_wait(&o_ready[b], (j >> 1) & 1);
-            ptx::tc_fence_after();
-            ptx::tmem_ld_32x16(taddr + ATC_O_COL0 + 32 * b + 16 * hh, o);
-            ptx::tmem_ld_wait();
-            ptx::tc_fence_before();
-            __syncwarp();
-            if (lane == 0) ptx::mbar_arrive(&o_free[b]);
-            const long long off = b ? out_off[1] : out_off[0];
-            if (off >= 0) {
-                const float inv = 1.0f / (xsum[(b * 2 + 0) * 128 + row] + xsum[(b * 2 + 1) * 128 + row]);
-                uint4* dst = reinterpret_cast<uint4*>(ctx + off + 16 * hh);
-#pragma unroll
-                for (int v4 = 0; v4 < 2; v4++) {
-                    uint4 ov;
-                    ov.x = pack2(__uint_as_float(o[8 * v4 + 0]) * inv, __uint_as_float(o[8 * v4 + 1]) * inv);
-                    ov.y = pack2(__uint_as_float(o[8 * v4 + 2]) * inv, __uint_as_float(o[8 * v4 + 3]) * inv);
-                    ov.z = pack2(__uint_as_float(o[8 * v4 + 4]) * inv, __uint_as_float(o[8 * v4 + 5]) * inv);
-                    ov.w = pack2(__uint_as_float(o[8 * v4 + 6]) * inv, __uint_as_float(o[8 * v4 + 7]) * inv);
-                    dst[v4] = ov;
-                }
-            }
-        };
-
-        int4 cur = n_it > 0 ? __ldg(&desc[blockIdx.x / heads]) : make_int4(0, 0, 0, 0);
-        for (int it = 0; it < n_it; it++) {
-            const int w = blockIdx.x + it * gridDim.x;
-            const int4 nxt = it + 1 < n_it ? __ldg(&desc[(w + gridDim.x) / heads]) : cur;
-            const int h = w % heads;
-            const int q0 = cur.z & 0xffff, lo = cur.z >> 16;
-            const int L = cur.y;
-            const int q = q0 + row;
-            const int nch = (skip_empty && (q0 + q4 * 32 >= L || q0 + q4 * 32 + 32 <= lo)) ? 0 : (L + 31) >> 5;
-            const int xb = (it & 1) * 2;
-            if (((L + 15) & ~15) > ATC_LONG) {  // the MMA warp waits for these before it may issue S(it)
-                pair_sync();                   // the partner's partial sums of item it - 1 are in shared memory
-                while (pend < it) readout(pend++);
-            }
-            ptx::mbar_wait(s_ready, it & 1);
-            ptx::tc_fence_after();
-            uint32_t r[32];
-            // pass 1: maximum over this warp's chunks, then over both warps of the row
-            float m = -INFINITY;
-            for (int c = hh; c < nch; c += 2) {
-                ptx::tmem_ld_32x32(taddr + c * 32, r);
-                ptx::tmem_ld_wait();
-                if (c * 32 + 32 <= L) {
-#pragma unroll
-                    for (int j = 0; j < 32; j++) m = fmaxf(m, __uint_as_float(r[j]));
-                } else {
-#pragma unroll
-                    for (int j = 0; j < 32; j++) m = (c * 32 + j < L) ? fmaxf(m, __uint_as_float(r[j])) : m;
-                }
-            }
-            xmax[(xb + hh) * 128 + row] = m;
-            pair_sync();  // also orders the partner's partial sums of item it - 1 before the read-out below
-            m = fmaxf(m, xmax[(xb + (hh ^ 1)) * 128 + row]);
-            // pass 2 in rounds of two chunks (one per warp)
-            const float ms = m * scale_log2;
-            float sum = 0.f;
-            for (int c0 = 0; c0 < nch; c0 += 2) {
-                const int c = c0 + hh;
-                const bool have = c < nch;
-                uint32_t pk[16];
-                if (have) {
-                    ptx::tmem_ld_32x32(taddr + c * 32, r);
-                    ptx::tmem_ld_wait();
-                    if (c * 32 + 32 <= L) {
-#pragma unroll
-                        for (int j = 0; j < 16; j++) {
-                            const float p0 = ex2f(fmaf(__uint_as_float(r[2 * j]), scale_log2, -ms));
-                            const float p1 = ex2f(fmaf(__uint_as_float(r[2 * j + 1]), scale_log2, -ms));
-                            sum += p0 + p1;
-                            pk[j] = pack2(p0, p1);
-                        }
-                    } else {
-#pragma unroll
-                        for (int j = 0; j < 16; j++) {
-                            float p0 = ex2f(fmaf(__uint_as_float(r[2 * j]), scale_log2, -ms));
-                            float p1 = ex2f(fmaf(__uint_as_float(r[2 * j + 1]), scale_log2, -ms));
-                            p0 = (c * 32 + 2 * j < L) ? p0 : 0.f;
-                            p1 = (c * 32 + 2 * j + 1 < L) ? p1 : 0.f;
-                            sum += p0 + p1;
-                            pk[j] = pack2(p0, p1);
-                        }
-                    }
-                }
-                pair_sync();  // both warps have read their chunk of this round: P may now cover the columns of S chunk c0 / 2
-                if (have) ptx::tmem_st_32x16(taddr + c * 16, pk);
-            }
-            xsum[(xb + hh) * 128 + row] = sum;
-            ptx::tmem_st_wait();
-            ptx::tc_fence_before();
-            __syncwarp();
-            if (lane == 0) ptx::mbar_arrive(p_ready);
-            const long long off = (q >= lo && q < L) ? static_cast<long long>(cur.x + q) * hidden + h * ATC_HD : -1;
-            if (it & 1) out_off[1] = off; else out_off[0] = off;
-            while (pend < it) readout(pend++);
-            cur = nxt;
-        }
-        pair_sync();  // the partner's partial sums of the last item
-        while (pend < n_it) readout(pend++);
-    }
-
     ptx::tc_fence_before();
     __syncthreads();
-    if (warp == SW + 1) {
+    if (warp == 5) {
         ptx::tc_fence_after();
         ptx::tmem_dealloc(tmem_base, ATC_TMEM_COLS);
     }
@@ -486,10 +341,7 @@ bool launch_attention_tc(cudaStream_t s, const __half* qkv, const int32_t* seq_s
     int4* desc = reinterpret_cast<int4*>(items);  // 2 descriptors per passage at most: fits the [n_seq * 8] int work-list buffer
     if (build_items) {  // once per encoder pass: the list is the same for every layer
         LB2_CUDA_OK(cudaMemsetAsync(item_count, 0, sizeof(int), s));
-        // LB2_ATTN_ROTATE = 1: second-block tails in a row quarter drawn per passage (A/B switch; measured neutral, default 0)
-        const char* rt = getenv("LB2_ATTN_ROTATE");
-        attention_tc_items_kernel<<<(n_seq + 255) / 256, 256, 0, s>>>(seq_start, seq_len, n_seq, row_base, desc, item_count,
-                                                                      rt ? atoi(rt) : 0);
+        attention_tc_items_kernel<<<(n_seq + 255) / 256, 256, 0, s>>>(seq_start, seq_len, n_seq, row_base, desc, item_count);
         LB2_CUDA_OK(cudaGetLastError());
     }
     CUtensorMap tm_qk, tm_v;
@@ -500,29 +352,12 @@ bool launch_attention_tc(cudaStream_t s, const __half* qkv, const int32_t* seq_s
     int dev = 0;
     cudaGetDevice(&dev);
     if (dev < 0 || dev >= 256 || !(attr_dev_mask[dev >> 5] & (1 << (dev & 31)))) {
-        LB2_CUDA_OK(cudaFuncSetAttribute(attention_tc_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, ATC_SMEM));
-        LB2_CUDA_OK(cudaFuncSetAttribute(attention_tc_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, ATC_SMEM));
+        LB2_CUDA_OK(cudaFuncSetAttribute(attention_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ATC_SMEM));
         if (dev >= 0 && dev < 256) attr_dev_mask[dev >> 5] |= 1 << (dev & 31);
     }
-    // LB2_ATTN_WAIT_NS > 0: the TMA and MMA warps sleep that long between mbarrier polls instead of spinning (A/B switch)
-    static const unsigned wait_ns = [] {
-        const char* e = getenv("LB2_ATTN_WAIT_NS");
-        return e ? static_cast<unsigned>(atoi(e)) : 0u;
-    }();
-    static const int skip_empty = [] {
-        const char* e = getenv("LB2_ATTN_SKIP");
-        return e ? atoi(e) : 1;
-    }();
-    // LB2_ATTN_WARPS = 4 (default) / 8 softmax warps per CTA (read per call: the tests compare the two).  Measured
-    // (profiles/r02c_attention_variants.log): 8 warps are 3-8 % SLOWER — the item time is set by the MUFU work of the two
-    // co-resident CTAs plus the softmax -> P.V -> S chain, not by latency hiding inside the softmax.
-    const char* sw = getenv("LB2_ATTN_WARPS");
-    if (!sw || atoi(sw) != 8)
-        attention_tc_kernel<4><<<2 * num_sms, ATC_THREADS, ATC_SMEM, s>>>(tm_qk, tm_v, desc, item_count, heads, hidden, ctx, wait_ns,
-                                                                         skip_empty);
-    else
-        attention_tc_kernel<8><<<2 * num_sms, ATC_THREADS8, ATC_SMEM, s>>>(tm_qk, tm_v, desc, item_count, heads, hidden, ctx,
-                                                                          wait_ns, skip_empty);
+    // Four softmax warps: eight (two per row quarter) measured 3-8 % slower (profiles/r02c_attention_variants.log) — the item
+    // time is set by the MUFU work of the two co-resident CTAs plus the softmax -> P.V -> S chain, not by latency hiding.
+    attention_tc_kernel<<<2 * num_sms, ATC_THREADS, ATC_SMEM, s>>>(tm_qk, tm_v, desc, item_count, heads, hidden, ctx);
     LB2_CUDA_OK(cudaGetLastError());
     return true;
 }

@@ -79,6 +79,8 @@ size_t encoder_weight_floats(const EncoderConfig& cfg);
 bool encoder_load(Encoder* enc, const EncoderConfig& cfg, const float* host_weights, size_t n_floats);
 void encoder_free(Encoder* enc);
 bool encoder_reserve(Encoder* enc, int64_t tokens, int64_t seqs);
+// whether each layer's residual projections fuse their LayerNorm (5 kernels per layer instead of 7)
+bool encoder_fuses_ln(const EncoderConfig& cfg);
 // Encode n_seq passages.  Passage i is node seq_node[i] of the token store (tok_store / tok_off,
 // device pointers); its rows in the packed activation matrix start at seq_start[i] - row_base;
 // n_tokens = packed row count.  Writes pooled (+normalised) fp32 embeddings to out[n_seq, H].

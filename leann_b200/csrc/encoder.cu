@@ -13,8 +13,6 @@
 
 #include <vector>
 
-#include <stdlib.h>
-
 #include "common.cuh"
 
 namespace lb2 {
@@ -414,8 +412,7 @@ bool launch_attention(cudaStream_t s, const __half* qkv, const int32_t* seq_star
     if (max_pos > 512) { set_error("attention: max_pos %d > 512", max_pos); return false; }
     // head_dim 32 and passages of at most 256 tokens (all-MiniLM-L6-v2): the tcgen05 kernel (attention_tc.cu).
     // Other shapes (bge-base: head_dim 64, up to 512 tokens) keep the mma.sync kernel below.
-    static const bool force_legacy = getenv("LB2_ATTN_LEGACY") && atoi(getenv("LB2_ATTN_LEGACY")) != 0;  // A/B profiling only
-    if (!force_legacy && attention_tc_supported(hidden, heads, max_pos)) {
+    if (attention_tc_supported(hidden, heads, max_pos)) {
         int dev = 0, sms = 148;
         cudaGetDevice(&dev);
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
@@ -611,6 +608,10 @@ bool encoder_reserve(Encoder* enc, int64_t tokens, int64_t seqs) {
     return true;
 }
 
+// hidden = 2 GEMM n-tiles (384): the residual projections carry their LayerNorm (gemm_f16_res_ln).  Other widths (bge-base,
+// 768) run the residual GEMM and the separate bandwidth-bound LayerNorm kernel.
+bool encoder_fuses_ln(const EncoderConfig& cfg) { return cfg.hidden == 2 * gemm_block_n(); }
+
 bool encoder_forward(Encoder* enc, cudaStream_t st, const uint16_t* tok_store, const uint64_t* tok_off,
                      const int32_t* seq_node, const int32_t* seq_start, int row_base, int n_seq, int n_tokens,
                      float* out) {
@@ -631,10 +632,7 @@ bool encoder_forward(Encoder* enc, cudaStream_t st, const uint16_t* tok_store, c
         prof_end(st, PROF_GEMM, 2.0 * T * (double)N * K);
         return ok;
     };
-    // hidden = 2 GEMM n-tiles: the residual projections carry their LayerNorm (gemm_f16_res_ln); LB2_FUSED_LN=0 keeps the
-    // separate bandwidth-bound LayerNorm kernel (A/B profiling).  hidden 768 (bge-base) always takes the unfused path.
-    static const bool fused_ln_env = !(getenv("LB2_FUSED_LN") && atoi(getenv("LB2_FUSED_LN")) == 0);
-    const bool fused_ln = fused_ln_env && H == 2 * gemm_block_n();
+    const bool fused_ln = encoder_fuses_ln(c);
     for (int l = 0; l < c.layers; l++) {
         const LayerWeights& w = enc->layers[l];
         if (!gemm(enc->x, &w.tm_qkv, w.w_qkv, w.b_qkv, nullptr, enc->qkv, 3 * H, H, EPI_BIAS, 3 * (H / c.heads))) return false;

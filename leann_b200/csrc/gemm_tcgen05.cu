@@ -17,7 +17,6 @@
 // between MMA and epilogue, so the epilogue of tile i overlaps the MMAs of tile i+1.
 // M is ragged (varlen-packed tokens): TMA zero-fills rows past M, stores are row-masked.
 #include <cuda_fp16.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 #include "ptx.cuh"
@@ -64,7 +63,7 @@ template <int BLOCK_N, int STAGES, int EPI>
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
 gemm_f16_tn_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
                    const __grid_constant__ CUtensorMap tmap_c, const __grid_constant__ CUtensorMap tmap_r,
-                   const float* __restrict__ bias, int M, int N, int K, int c_group, int wait_ns, int pf_tiles) {
+                   const float* __restrict__ bias, int M, int N, int K, int c_group) {
     using L = GemmSmem<BLOCK_N, STAGES>;
     constexpr int TMEM_COLS = (2 * BLOCK_N <= 32) ? 32 : (2 * BLOCK_N <= 64) ? 64 : (2 * BLOCK_N <= 128) ? 128
                             : (2 * BLOCK_N <= 256) ? 256 : 512;
@@ -121,16 +120,10 @@ gemm_f16_tn_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
         for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
             const int m_blk = tile / num_n, n_blk = tile % num_n;
             for (int kb = 0; kb < num_k; kb++) {
-                // the A k-block this CTA loads `pf_tiles` k-blocks from now: into L2 (of the num_n CTAs that read a row
-                // block at about the same time, the one working on column block 0 asks)
-                const int pf_it = (kb + pf_tiles) / num_k, pf_kb = (kb + pf_tiles) - pf_it * num_k;
-                const int pf_tile = tile + pf_it * gridDim.x;
-                const bool pf = pf_tiles > 0 && pf_tile < num_tiles && pf_tile % num_n == 0;
-                ptx::mbar_wait_ns(&empty_bar[stage], phase ^ 1, wait_ns * 8);
+                ptx::mbar_wait(&empty_bar[stage], phase ^ 1);
                 uint8_t* sa = smem + stage * L::STAGE_BYTES;
                 uint8_t* sb = sa + L::A_BYTES;
                 if (ptx::elect_one()) {
-                    if (pf) ptx::tma_prefetch_2d(&tmap_a, pf_kb * BLOCK_K, (pf_tile / num_n) * BLOCK_M);
                     ptx::mbar_expect_tx(&full_bar[stage], L::STAGE_BYTES);
                     ptx::tma_load_2d(sa, &tmap_a, &full_bar[stage], kb * BLOCK_K, m_blk * BLOCK_M);
                     ptx::tma_load_2d(sb, &tmap_b, &full_bar[stage], kb * BLOCK_K, n_blk * BLOCK_N);
@@ -203,7 +196,7 @@ gemm_f16_tn_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
                         ptx::tma_load_2d(stage_buf + c * 2048, &tmap_r, &res_bar[ew], colbase + c * 32, row0);
                 }
             }
-            ptx::mbar_wait_ns(&tmem_full[as], aphase, wait_ns);
+            ptx::mbar_wait(&tmem_full[as], aphase);
             ptx::tc_fence_after();
             const uint32_t taddr = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16) + as * BLOCK_N + half * NCH * 32;
             uint32_t r[2][32];
@@ -298,6 +291,16 @@ gemm_f16_tn_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
 // drains the MMAs that read the old panel (b_empty) and reloads.  Epilogue as in gemm_f16_tn_kernel (bias / GELU -> fp16
 // -> swizzled 32x32 box -> TMA store), one staging box per warp (reused per chunk: the box is free again long before the
 // next chunk's arithmetic is done), bias panel in shared memory.
+//
+// How many k-blocks ahead of its loads the producer asks L2 for the activation rows (cp.async.bulk.prefetch.tensor).  The
+// shared-memory ring only covers 4 k-blocks = ~1 500 tensor clocks of work, while a TMA load of rows that are not in L2 yet
+// takes ~3 000 clocks under load (ncu: the MMA warp spent 42 % of its samples on the `full` barriers); the prefetch turns
+// those loads into L2 hits without spending shared memory (12 k-blocks x 16 KB x 148 CTAs = 28 MB outstanding, L2 is 126 MB).
+// Measured (profiles/r02c_gemm_prefetch_sweep.log): the weight-stationary kernel gains 3-4 % on the QKV shape with 6-12
+// k-blocks, nothing on FFN-up; the streaming kernels (which also stream W) LOSE 10-30 % at K = 1536 — their prefetches
+// compete with the loads they are meant to help — so only the weight-stationary kernel prefetches.
+constexpr int WS_PF_TILES = 12;
+
 template <int BLOCK_N, int NUM_K, int STAGES>
 struct GemmWsSmem {
     static constexpr int A_BYTES = BLOCK_M * BLOCK_K * 2;       // one k-block of activations
@@ -315,7 +318,7 @@ template <int BLOCK_N, int NUM_K, int STAGES, int EPI>
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
 gemm_f16_ws_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
                    const __grid_constant__ CUtensorMap tmap_c, const float* __restrict__ bias, int M, int N, int c_group,
-                   int ctas_per_panel, int pf_tiles, int direct_store, __half* __restrict__ C) {
+                   int ctas_per_panel) {
     using L = GemmWsSmem<BLOCK_N, NUM_K, STAGES>;
     static_assert(L::TOTAL <= 232448, "shared memory budget");
     static_assert(EPI == EPI_BIAS || EPI == EPI_BIAS_GELU, "no residual variant");
@@ -398,10 +401,10 @@ gemm_f16_ws_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
                 cur_n = n_blk;
             }
             for (int kb = 0; kb < NUM_K; kb++) {
-                // the A k-block this CTA loads `pf_tiles` k-blocks from now: into L2 (only the CTAs of panel 0 ask — the
+                // the A k-block this CTA loads WS_PF_TILES k-blocks from now: into L2 (only the CTAs of panel 0 ask — the
                 // others read the same rows at the same time)
-                const int pf_it = (kb + pf_tiles) / NUM_K, pf_kb = (kb + pf_tiles) - pf_it * NUM_K;
-                const bool pf = pf_tiles > 0 && n_blk == 0 && tile + pf_it < t_end;
+                const int pf_it = (kb + WS_PF_TILES) / NUM_K, pf_kb = (kb + WS_PF_TILES) - pf_it * NUM_K;
+                const bool pf = n_blk == 0 && tile + pf_it < t_end;
                 ptx::mbar_wait(&empty_bar[stage], phase ^ 1);
                 if (ptx::elect_one()) {
                     if (pf) ptx::tma_prefetch_2d(&tmap_a, pf_kb * BLOCK_K, (m_blk + pf_it) * BLOCK_M);
@@ -512,26 +515,6 @@ gemm_f16_ws_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
                     for (int u = 0; u < 4; u++) oh[u] = __floats2half2_rn(v[2 * u], v[2 * u + 1]);
                 }
                 uint8_t* box = box_base + lane * 64;
-                if (direct_store) {
-                    // direct stores (LB2_GEMM_WS_DIRECT_STORE=1; measured 5-9 % slower than the TMA stores, kept as a tested alternative): the box only transposes (thread = row  ->  4 lanes = one 64-byte row segment), the
-                    // warp writes 8 rows x 64 B per instruction itself; no TMA store, no async-proxy fence, no wait for the
-                    // TMA unit to have read the box
-                    __syncwarp();  // the previous chunk's reads of the box are done
-#pragma unroll
-                    for (int j4 = 0; j4 < 4; j4++) *reinterpret_cast<uint4*>(box + ((j4 ^ swz) << 4)) = ov[j4];
-                    __syncwarp();
-                    const int piece = lane & 3;
-                    __half* cbase = c_group > 0 ? C + (static_cast<size_t>(col0 / c_group) * M) * c_group + col0 % c_group
-                                                : C + col0;
-                    const size_t pitch = c_group > 0 ? c_group : N;
-#pragma unroll
-                    for (int i = 0; i < 4; i++) {
-                        const int r = 8 * i + (lane >> 2);
-                        const uint4 v = *reinterpret_cast<const uint4*>(box_base + r * 64 + ((piece ^ ((r >> 1) & 3)) << 4));
-                        if (row0 + r < M) *reinterpret_cast<uint4*>(cbase + (row0 + r) * pitch + piece * 8) = v;
-                    }
-                    continue;
-                }
                 // the store issued from this warp's box one chunk ago must have finished reading it
                 if (lane == 0) ptx::bulk_wait_read<0>();
                 __syncwarp();
@@ -599,7 +582,7 @@ template <int BLOCK_N, int STAGES, bool PAIR>
 __device__ __forceinline__ void
 gemm_f16_ln_body(const CUtensorMap& tmap_a, const CUtensorMap& tmap_b, const CUtensorMap& tmap_c, const CUtensorMap& tmap_r,
                  const float* __restrict__ bias, const float* __restrict__ gamma, const float* __restrict__ beta, float eps,
-                 int M, int K, int wait_ns, int pf_tiles) {
+                 int M, int K) {
     using L = GemmLnSmem<BLOCK_N, STAGES, PAIR>;
     const int rank = PAIR ? static_cast<int>(ptx::cluster_ctarank()) : 0;
     // row blocks are dealt to CTAs (pairs: to the pair, rank r takes the r-th of two consecutive ones; a block past the end
@@ -662,16 +645,10 @@ gemm_f16_ln_body(const CUtensorMap& tmap_a, const CUtensorMap& tmap_b, const CUt
         for (int m_blk = blk_first; m_blk < num_m + rank; m_blk += blk_step) {
             for (int n_blk = 0; n_blk < 2; n_blk++) {
                 for (int kb = 0; kb < num_k; kb++) {
-                    // the A k-block this CTA loads `pf_tiles` first-pass k-blocks from now: into L2 (the second column half
-                    // re-reads what the first one loaded)
-                    const int pf_it = (kb + pf_tiles) / num_k, pf_kb = (kb + pf_tiles) - pf_it * num_k;
-                    const int pf_blk = m_blk + pf_it * blk_step;
-                    const bool pf = pf_tiles > 0 && n_blk == 0 && pf_blk < num_m;
-                    ptx::mbar_wait_ns(&empty_bar[stage], phase ^ 1, wait_ns * 8);
+                    ptx::mbar_wait(&empty_bar[stage], phase ^ 1);
                     uint8_t* sa = smem + stage * L::STAGE_BYTES;
                     uint8_t* sb = sa + L::A_BYTES;
                     if (ptx::elect_one()) {
-                        if (pf) ptx::tma_prefetch_2d(&tmap_a, pf_kb * BLOCK_K, pf_blk * BLOCK_M);
                         if (PAIR) {
                             // both CTAs' bytes complete on rank 0's barrier; rank 0 announces the total
                             if (rank == 0) ptx::mbar_expect_tx(&full_bar[stage], 2 * L::STAGE_BYTES);
@@ -754,7 +731,7 @@ gemm_f16_ln_body(const CUtensorMap& tmap_a, const CUtensorMap& tmap_b, const CUt
             for (int n_blk = 0; n_blk < 2; n_blk++) {
                 uint8_t* boxes = smem + L::EPI_OFFSET + n_blk * L::TILE_BOX_BYTES + ew * NCH * 2048;
                 const int colbase = n_blk * BLOCK_N + half * NCH * 32;
-                ptx::mbar_wait_ns(&tmem_full[n_blk], it & 1, wait_ns);
+                ptx::mbar_wait(&tmem_full[n_blk], it & 1);
                 ptx::tc_fence_after();
                 const uint32_t taddr = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16) + n_blk * BLOCK_N + half * NCH * 32;
                 uint32_t r[2][32];
@@ -856,8 +833,8 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
 gemm_f16_ln_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
                    const __grid_constant__ CUtensorMap tmap_c, const __grid_constant__ CUtensorMap tmap_r,
                    const float* __restrict__ bias, const float* __restrict__ gamma, const float* __restrict__ beta, float eps,
-                   int M, int K, int wait_ns, int pf_tiles) {
-    gemm_f16_ln_body<BLOCK_N, STAGES, false>(tmap_a, tmap_b, tmap_c, tmap_r, bias, gamma, beta, eps, M, K, wait_ns, pf_tiles);
+                   int M, int K) {
+    gemm_f16_ln_body<BLOCK_N, STAGES, false>(tmap_a, tmap_b, tmap_c, tmap_r, bias, gamma, beta, eps, M, K);
 }
 
 template <int BLOCK_N, int STAGES>
@@ -865,8 +842,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(GEMM_THREADS, 1)
 gemm_f16_ln_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
                         const __grid_constant__ CUtensorMap tmap_c, const __grid_constant__ CUtensorMap tmap_r,
                         const float* __restrict__ bias, const float* __restrict__ gamma, const float* __restrict__ beta,
-                        float eps, int M, int K, int wait_ns, int pf_tiles) {
-    gemm_f16_ln_body<BLOCK_N, STAGES, true>(tmap_a, tmap_b, tmap_c, tmap_r, bias, gamma, beta, eps, M, K, wait_ns, pf_tiles);
+                        float eps, int M, int K) {
+    gemm_f16_ln_body<BLOCK_N, STAGES, true>(tmap_a, tmap_b, tmap_c, tmap_r, bias, gamma, beta, eps, M, K);
 }
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
@@ -957,31 +934,8 @@ static bool make_tmap_f16_grouped(CUtensorMap* map, const void* ptr, uint64_t ro
     return true;
 }
 
-// sleep between mbarrier polls of the producer (x8) and the epilogue warps; 0 = spin.  LB2_GEMM_WAIT_NS overrides (A/B runs).
-static int gemm_wait_ns() {
-    static const int v = getenv("LB2_GEMM_WAIT_NS") ? atoi(getenv("LB2_GEMM_WAIT_NS")) : 0;
-    return v;
-}
-
 constexpr int GEMM_BLOCK_N = 192;
 constexpr int GEMM_STAGES = 4;
-
-// How many k-blocks ahead of its loads the producer asks L2 for the activation rows (cp.async.bulk.prefetch.tensor).  The
-// shared-memory ring only covers 4 k-blocks = ~1 500 tensor clocks of work, while a TMA load of rows that are not in L2 yet
-// takes ~3 000 clocks under load (ncu: the MMA warp spent 42 % of its samples on the `full` barriers); the prefetch turns
-// those loads into L2 hits without spending shared memory (12 k-blocks x 16 KB x 148 CTAs = 28 MB outstanding, L2 is 126 MB).
-// Measured (profiles/r02c_gemm_prefetch_sweep.log): the weight-stationary kernel gains 3-4 % on the QKV shape with 6-12
-// k-blocks, nothing on FFN-up; the streaming kernels (which also stream W) LOSE 10-30 % at K = 1536 — their prefetches
-// compete with the loads they are meant to help — so only the weight-stationary kernel prefetches by default.
-// LB2_GEMM_PF / LB2_GEMM_PF_STREAM override (0 = off).
-static int gemm_prefetch_tiles() {
-    static const int v = getenv("LB2_GEMM_PF") ? atoi(getenv("LB2_GEMM_PF")) : 12;
-    return v;
-}
-static int gemm_prefetch_tiles_stream() {
-    static const int v = getenv("LB2_GEMM_PF_STREAM") ? atoi(getenv("LB2_GEMM_PF_STREAM")) : 0;
-    return v;
-}
 
 template <int EPI>
 static cudaError_t launch_gemm(cudaStream_t stream, const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& tc,
@@ -998,23 +952,19 @@ static cudaError_t launch_gemm(cudaStream_t stream, const CUtensorMap& ta, const
     }
     const int tiles = ((M + BLOCK_M - 1) / BLOCK_M) * (N / GEMM_BLOCK_N);
     const int grid = tiles < num_sms ? tiles : num_sms;
-    kern<<<grid, GEMM_THREADS, L::TOTAL, stream>>>(ta, tb, tc, tr, bias, M, N, K, c_group, gemm_wait_ns(), gemm_prefetch_tiles_stream());
+    kern<<<grid, GEMM_THREADS, L::TOTAL, stream>>>(ta, tb, tc, tr, bias, M, N, K, c_group);
     return cudaGetLastError();
 }
 
-// weight-stationary kernel for K = 384 (LB2_GEMM_WS=0 falls back to the streaming kernel)
+// weight-stationary kernel for K = 384
 constexpr int WS_NUM_K = 6;
 constexpr int WS_STAGES = 4;
-static bool gemm_ws_enabled() {
-    static const bool v = !(getenv("LB2_GEMM_WS") && atoi(getenv("LB2_GEMM_WS")) == 0);
-    return v;
-}
 
-template <int EPI, int WS_STAGES_T>
-static cudaError_t launch_gemm_ws_s(cudaStream_t stream, const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& tc,
-                                  const float* bias, int M, int N, int c_group, int num_sms, __half* C) {
-    using L = GemmWsSmem<GEMM_BLOCK_N, WS_NUM_K, WS_STAGES_T>;
-    auto kern = gemm_f16_ws_kernel<GEMM_BLOCK_N, WS_NUM_K, WS_STAGES_T, EPI>;
+template <int EPI>
+static cudaError_t launch_gemm_ws(cudaStream_t stream, const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& tc,
+                                  const float* bias, int M, int N, int c_group, int num_sms) {
+    using L = GemmWsSmem<GEMM_BLOCK_N, WS_NUM_K, WS_STAGES>;
+    auto kern = gemm_f16_ws_kernel<GEMM_BLOCK_N, WS_NUM_K, WS_STAGES, EPI>;
     static thread_local int attr_dev_mask[8] = {0};
     int dev = 0;
     cudaGetDevice(&dev);
@@ -1027,25 +977,12 @@ static cudaError_t launch_gemm_ws_s(cudaStream_t stream, const CUtensorMap& ta, 
     int cpp = num_sms / num_n;  // CTAs per panel
     if (cpp > num_m) cpp = num_m;
     int grid = cpp * num_n;
-    const char* ff = getenv("LB2_GEMM_WS_FREEFORM");  // test hook: exercise the panel-change path
-    if (ff && atoi(ff) != 0) cpp = 0;
     if (cpp == 0) {  // more panels than SMs: free-form split of the tile list
         const long long tiles = static_cast<long long>(num_m) * num_n;
         grid = tiles < num_sms ? static_cast<int>(tiles) : num_sms;
     }
-    kern<<<grid, GEMM_THREADS, L::TOTAL, stream>>>(ta, tb, tc, bias, M, N, c_group, cpp, gemm_prefetch_tiles(),
-                                                    getenv("LB2_GEMM_WS_DIRECT_STORE") ? atoi(getenv("LB2_GEMM_WS_DIRECT_STORE")) : 0, C);
+    kern<<<grid, GEMM_THREADS, L::TOTAL, stream>>>(ta, tb, tc, bias, M, N, c_group, cpp);
     return cudaGetLastError();
-}
-
-// LB2_GEMM_WS_STAGES = 2 / 3 selects a shallower activation ring (depth-sensitivity experiment); default 4
-template <int EPI>
-static cudaError_t launch_gemm_ws(cudaStream_t stream, const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& tc,
-                                  const float* bias, int M, int N, int c_group, int num_sms, __half* C) {
-    static const int st = getenv("LB2_GEMM_WS_STAGES") ? atoi(getenv("LB2_GEMM_WS_STAGES")) : WS_STAGES;
-    if (st == 2) return launch_gemm_ws_s<EPI, 2>(stream, ta, tb, tc, bias, M, N, c_group, num_sms, C);
-    if (st == 3) return launch_gemm_ws_s<EPI, 3>(stream, ta, tb, tc, bias, M, N, c_group, num_sms, C);
-    return launch_gemm_ws_s<EPI, WS_STAGES>(stream, ta, tb, tc, bias, M, N, c_group, num_sms, C);
 }
 
 // A [M,K] fp16 row-major, W [N,K] fp16 row-major (nn.Linear layout), C [M,N] fp16.
@@ -1078,9 +1015,9 @@ bool gemm_f16(cudaStream_t stream, const __half* A, const CUtensorMap* tmap_w, c
         tmap_w = &tb_local;
     }
     cudaError_t e;
-    if (K == WS_NUM_K * BLOCK_K && epi != EPI_BIAS_RES && gemm_ws_enabled()) {
-        e = epi == EPI_BIAS ? launch_gemm_ws<EPI_BIAS>(stream, ta, *tmap_w, tc, bias, M, N, c_group, num_sms, C)
-                            : launch_gemm_ws<EPI_BIAS_GELU>(stream, ta, *tmap_w, tc, bias, M, N, c_group, num_sms, C);
+    if (K == WS_NUM_K * BLOCK_K && epi != EPI_BIAS_RES) {
+        e = epi == EPI_BIAS ? launch_gemm_ws<EPI_BIAS>(stream, ta, *tmap_w, tc, bias, M, N, c_group, num_sms)
+                            : launch_gemm_ws<EPI_BIAS_GELU>(stream, ta, *tmap_w, tc, bias, M, N, c_group, num_sms);
         if (e != cudaSuccess) {
             set_error("gemm_f16 (weight-stationary) launch: %s", cudaGetErrorString(e));
             return false;
@@ -1100,14 +1037,8 @@ bool gemm_f16(cudaStream_t stream, const __half* A, const CUtensorMap* tmap_w, c
     return true;
 }
 
-// CTA-pair (cta_group::2) variant of the fused-LayerNorm projection, the default; LB2_GEMM_LN_PAIR=0 selects the single-CTA
-// kernel (read per call: the tests flip it)
-static bool gemm_ln_pair_enabled() {
-    const char* e = getenv("LB2_GEMM_LN_PAIR");
-    return e ? atoi(e) != 0 : true;
-}
-
-// x_out[M, 384] = LayerNorm(A[M, K] . W[384, K]^T + bias + residual) * gamma + beta  (gemm_f16_ln_kernel)
+// x_out[M, 384] = LayerNorm(A[M, K] . W[384, K]^T + bias + residual) * gamma + beta: gemm_f16_ln_pair_kernel (CTA pairs)
+// for two row blocks or more, gemm_f16_ln_kernel (one CTA) for a single row block
 bool gemm_f16_res_ln(cudaStream_t stream, const __half* A, const CUtensorMap* tmap_w, const __half* W, const float* bias,
                      const __half* residual, const float* gamma, const float* beta, float eps, __half* C, int M, int N, int K,
                      int num_sms) {
@@ -1124,7 +1055,7 @@ bool gemm_f16_res_ln(cudaStream_t stream, const __half* A, const CUtensorMap* tm
     int dev = 0;
     cudaGetDevice(&dev);
     const bool dev_ok = dev >= 0 && dev < 256;
-    if (gemm_ln_pair_enabled() && num_m >= 2) {
+    if (num_m >= 2) {
         // CTA pairs (cta_group::2): each CTA loads half of the W rows of a panel -> its own tensor map (96-row boxes)
         constexpr int PAIR_STAGES = 4;
         using L = GemmLnSmem<GEMM_BLOCK_N, PAIR_STAGES, true>;
@@ -1149,8 +1080,7 @@ bool gemm_f16_res_ln(cudaStream_t stream, const __half* A, const CUtensorMap* tm
         int pairs = dev_ok ? max_clusters[dev] : num_sms / 2;  // co-resident pairs: the kernel is persistent
         if (pairs > num_sms / 2) pairs = num_sms / 2;
         if (pairs > (num_m + 1) / 2) pairs = (num_m + 1) / 2;
-        kern<<<2 * pairs, GEMM_THREADS, L::TOTAL, stream>>>(ta, tb_local, tc, tr, bias, gamma, beta, eps, M, K, gemm_wait_ns(),
-                                                             gemm_prefetch_tiles_stream());
+        kern<<<2 * pairs, GEMM_THREADS, L::TOTAL, stream>>>(ta, tb_local, tc, tr, bias, gamma, beta, eps, M, K);
         cudaError_t e = cudaGetLastError();
         if (e != cudaSuccess) { set_error("gemm_f16_res_ln (pair) launch: %s", cudaGetErrorString(e)); return false; }
         return true;
@@ -1169,7 +1099,7 @@ bool gemm_f16_res_ln(cudaStream_t stream, const __half* A, const CUtensorMap* tm
         if (dev_ok) attr_dev_mask[dev >> 5] |= 1 << (dev & 31);
     }
     const int grid = num_m < num_sms ? num_m : num_sms;
-    kern<<<grid, GEMM_THREADS, L::TOTAL, stream>>>(ta, *tmap_w, tc, tr, bias, gamma, beta, eps, M, K, gemm_wait_ns(), gemm_prefetch_tiles_stream());
+    kern<<<grid, GEMM_THREADS, L::TOTAL, stream>>>(ta, *tmap_w, tc, tr, bias, gamma, beta, eps, M, K);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) { set_error("gemm_f16_res_ln launch: %s", cudaGetErrorString(e)); return false; }
     return true;

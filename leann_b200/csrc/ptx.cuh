@@ -53,30 +53,6 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
         : "memory");
 }
 
-// Polite wait for warps that share an SM sub-partition with compute warps: between polls the thread sleeps, so the spin
-// does not eat the issue slots of the warps it is waiting for (ncu: two control warps per CTA polling back to back executed
-// 40 % of all instructions of the attention kernel).
-__device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t"
-        ".reg .pred P1;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 P1, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, P1;\n\t"
-        "}\n"
-        : "=r"(ok)
-        : "r"(smem_u32(bar)), "r"(parity)
-        : "memory");
-    return ok != 0;
-}
-__device__ __forceinline__ void mbar_wait_sleep(uint64_t* bar, uint32_t parity, unsigned ns) {
-    while (!mbar_try_wait(bar, parity)) __nanosleep(ns);
-}
-// ns == 0: plain spin (latency-critical waits)
-__device__ __forceinline__ void mbar_wait_ns(uint64_t* bar, uint32_t parity, unsigned ns) {
-    if (ns == 0) mbar_wait(bar, parity); else mbar_wait_sleep(bar, parity, ns);
-}
-
 // ---------------------------------------------------------------- TMA
 __device__ __forceinline__ void prefetch_tmap(const CUtensorMap* m) {
     asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(m)) : "memory");

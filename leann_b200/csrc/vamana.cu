@@ -21,7 +21,6 @@
 
 #include <algorithm>
 #include <cfloat>
-#include <cstdlib>
 
 namespace lb2 {
 
@@ -388,8 +387,8 @@ int pick_warps(const VamanaWork& w) {
 // ncu shows 65 GB of DRAM reads for 2.6 GB of algorithmic bytes (profiles/r01e_traversal_ncu.md).  Capping the
 // in-flight tables to an L2-sized budget was measured and is SLOWER (1 M points, 154-byte codes: 64 MB -> 2.5e5 q/s,
 // 128 MB -> 2.8e5, no cap -> 4.9e5; profiles/r01e_vamana_l2_budget_sweep.log): the kernel is bound by the latency of
-// its dependent gathers, and thousands of warps hide it better than L2 hits do.  The cap therefore stays off unless
-// LB2_VAMANA_L2_MB is set; DESIGN.md section 7 discusses the shared-memory-table variant.
+// its dependent gathers, and thousands of warps hide it better than L2 hits do, so every slot is used.  DESIGN.md
+// section 7 discusses the shared-memory-table variant.
 void vamana_plan(const DevVamana& v, VamanaWork& w, int num_sms) {
     int warps = pick_warps(w);
     size_t smem = search_smem(w, warps);
@@ -398,15 +397,7 @@ void vamana_plan(const DevVamana& v, VamanaWork& w, int num_sms) {
     int blocks = 0;
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks, vamana_search_kernel, warps * 32, smem) != cudaSuccess || blocks < 1)
         blocks = 1;
-    long long slots = (long long)num_sms * blocks * warps;
-    const long long lut_bytes = (long long)v.n_chunks * 256 * (long long)sizeof(float);
-    long long budget_mb = 1ll << 40;  // off
-    if (const char* e = getenv("LB2_VAMANA_L2_MB")) budget_mb = std::max(1, atoi(e));  // tuning knob for experiments
-    const long long cap = std::max<long long>(num_sms, (budget_mb << 20) / lut_bytes);
-    if (cap < slots) {
-        while (warps > 1 && cap / warps < 2 * num_sms) warps >>= 1;  // at least two blocks per SM before widening blocks
-        slots = std::max<long long>(1, cap / warps) * warps;
-    }
+    const long long slots = (long long)num_sms * blocks * warps;
     w.warps = warps;
     w.slots = (int)slots;
 }

@@ -37,12 +37,9 @@ print(f"hnsw stored: {NQ/(st.gpu_ms/1e3):.0f} q/s, recall {recall_at_k(I, gt):.3
 idx.close()
 prefix, vg, coords, pq, codes, mx = build_diskann_index(work, "da", E.cpu().numpy(), metric="mips", R=32, partition=True, keep_disk_index=False)
 da = capi.DiskannIndex(prefix, "mips", prefix, 0)
-import os
-for mb in ([int(x) for x in os.environ.get("SWEEP_L2_MB", "").split(",") if x] or [64]):
-  os.environ["LB2_VAMANA_L2_MB"] = str(mb)
-  for _ in range(2):
+for _ in range(2):
     D, I = da.search(Q, 10, capi.make_diskann_params(64, 1, recompute_embeddings=False, skip_search_reorder=True))
-  st = da.last_stats
-  byts = st.n_requested * (4 * 32 + 4) + st.ndis * pq.n_chunks
-  print(f"[L2 budget {mb} MB] vamana pq-only: {NQ/(st.gpu_ms/1e3):.0f} q/s, recall(pq order) {recall_at_k(I, gt):.3f}, {st.n_requested/NQ:.0f} expansions, {st.ndis/NQ:.0f} PQ comparisons per query, "
-        f"{pq.n_chunks} B codes; algorithmic {byts/1e6:.1f} MB per launch -> {byts/(st.gpu_ms/1e3)/1e9:.0f} GB/s", flush=True)
+st = da.last_stats
+byts = st.n_requested * (4 * 32 + 4) + st.ndis * pq.n_chunks
+print(f"vamana pq-only: {NQ/(st.gpu_ms/1e3):.0f} q/s, recall(pq order) {recall_at_k(I, gt):.3f}, {st.n_requested/NQ:.0f} expansions, {st.ndis/NQ:.0f} PQ comparisons per query, "
+      f"{pq.n_chunks} B codes; algorithmic {byts/1e6:.1f} MB per launch -> {byts/(st.gpu_ms/1e3)/1e9:.0f} GB/s", flush=True)
